@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          # ours (N > 1: launched by torchrun)
     python bench.py --impl reference [...]                       # the reference's CPU path (oracle port)
+    python bench.py [...] --dump-outputs DIR                     # + the last timed step's fingerprints as DIR/*.npy
 
 Primary line = BASELINE.json metric part (i), domain fingerprints/s, on configs[1]:
   100k synthetic domains, L ~ U{40..500}, two ESM-2 layers x 1280 fp32.  A step is one batch of
@@ -221,6 +222,23 @@ def traffic_for(kernel):
     return None
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, out):
+    """--dump-outputs: the int8 fingerprints [domains, 480] that the last timed step wrote, as DIR/fingerprints.npy in
+    float32.  The inputs come from fixed seeds, so two builds run with the same arguments can be compared row for row.
+    Above DUMP_BYTES a fixed, seeded sample of rows is kept and their positions go to DIR/fingerprint_rows.npy."""
+    a = out.cpu().numpy().astype(np.float32)
+    os.makedirs(path, exist_ok=True)
+    if a.nbytes > DUMP_BYTES:
+        keep = (DUMP_BYTES - (1 << 16)) // (a.shape[1] * 4 + 8)
+        rows = np.sort(np.random.RandomState(0).choice(a.shape[0], keep, replace=False))
+        a = a[rows]
+        np.save(os.path.join(path, 'fingerprint_rows.npy'), rows.astype(np.float64))
+    np.save(os.path.join(path, 'fingerprints.npy'), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -295,6 +313,8 @@ def run_ours(args):
         evs[i + 1].record()
     barrier()
     launches = int(L.dctd_launch_count(0))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pool[(args.warmup + args.steps - 1) % len(pool)][2])
     total_ms = evs[0].elapsed_time(evs[-1])
     per_step = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]
     algo = [pool[(args.warmup + i) % len(pool)][0].algorithmic_bytes for i in range(args.steps)]
@@ -1052,7 +1072,13 @@ def main():
     ap.add_argument('--no-dctsim', action='store_true')
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-fused', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the fingerprints of the last timed step to DIR/*.npy (float32), for comparing two builds')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
     if args.impl == 'reference':
         run_reference(args)

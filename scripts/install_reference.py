@@ -1,9 +1,11 @@
-"""Installs the UNMODIFIED reference modules into git-ignored baseline/_ref/ (they travel to the GPU box with the
-snapshot): the reference has no installable package (its pyproject.toml lists build requirements only), so the
-"install" is a verbatim copy of /root/reference/src/*.py plus a manifest of their sha256 digests.  Used by
-  * bench.py --impl reference   (the reference's own Fingerprint.quantize under multiprocessing.Pool), and
-  * tests/test_reference_dropin_gpu.py (the reference's Database / search_db running on the faiss shim).
-Nothing under dctdomain_b200/ imports it.  No-op when /root/reference is absent (GPU box: the copy already exists)."""
+"""Installs the UNMODIFIED reference modules into git-ignored baseline/_ref/ for `bench.py --impl reference` (the
+reference's own Fingerprint.quantize under multiprocessing.Pool; without the copy an oracle port stands in):
+
+    python scripts/install_reference.py <reference checkout>      (or DCTD_REFERENCE=<reference checkout>)
+
+The reference has no installable package (its pyproject.toml lists build requirements only), so the "install" is a
+verbatim copy of <checkout>/src/*.py plus a manifest of their sha256 digests.  Nothing under dctdomain_b200/ or tests/
+imports it."""
 import hashlib
 import json
 import os
@@ -11,15 +13,18 @@ import shutil
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SRC = os.environ.get('DCTD_REFERENCE', '/root/reference')
 DST = os.path.join(ROOT, 'baseline', '_ref')
 
 
 def main():
-    src = os.path.join(SRC, 'src')
+    ref = sys.argv[1] if len(sys.argv) > 1 else os.environ.get('DCTD_REFERENCE')
+    if not ref:
+        print(__doc__)
+        return 2
+    src = os.path.join(ref, 'src')
     if not os.path.isdir(src):
         print(f'{src} not present: baseline/_ref left as it is')
-        return 0
+        return 1
     os.makedirs(DST, exist_ok=True)
     manifest = {}
     for name in sorted(os.listdir(src)):
