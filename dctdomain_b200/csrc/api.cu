@@ -10,7 +10,12 @@
 namespace dctd {
 static thread_local cudaError_t g_last_cuda = cudaSuccess;
 static thread_local int64_t g_launches = 0;
-void set_cuda_error(cudaError_t e) { g_last_cuda = e; }
+void set_cuda_error(cudaError_t e) {
+    g_last_cuda = e;
+    // a failed runtime call also leaves its (non-sticky) error pending in the runtime; consume it, or the launch check of
+    // the next, valid call - ours or the caller's - would report it as its own
+    (void)cudaGetLastError();
+}
 void count_launch(int n) { g_launches += n; }
 }  // namespace dctd
 

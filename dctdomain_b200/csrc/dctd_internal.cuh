@@ -6,7 +6,7 @@
 
 namespace dctd {
 
-void set_cuda_error(cudaError_t e);   // records into the thread-local "last CUDA error"
+void set_cuda_error(cudaError_t e);   // records into the thread-local "last CUDA error", clears the runtime's pending one
 void count_launch(int n = 1);         // bumps the thread-local launch counter
 
 #define DCTD_CUDA_TRY(expr)                      \

@@ -1533,6 +1533,11 @@ int dctd_fp_execute(const dctd_fp_plan *plan, const void *const *h_src_ptrs, int
     } else if (K == 2 && ldc && plan->D == 2560 && prm.lay.RL == 1) fn = fp_kernel<2, 4, 8, kMaxThreads, 1, 2560, 1>;
     else fn = pick_k<4, 8, kMaxThreads, 1>(K);
     if (!fn) return DCTD_ERR_UNSUPPORTED;
+    // the opt-in limit bounds static + dynamic shared memory: fp_kernel's static variables (176 B) can tip a layout that
+    // passed the check above over it (D = 5072 at n = 3, m = 80), and cudaFuncSetAttribute would then fail
+    cudaFuncAttributes fa{};
+    DCTD_CUDA_TRY(cudaFuncGetAttributes(&fa, fn));
+    if (prm.lay.smem + fa.sharedSizeBytes > (size_t)max_smem) return DCTD_ERR_UNSUPPORTED;
     DCTD_CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prm.lay.smem));
     int per_sm = 0;
     DCTD_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, prm.lay.T, prm.lay.smem));

@@ -153,7 +153,11 @@ int dctd_fp_plan_dump_records(const dctd_fp_plan *plan, int32_t *records, int64_
 /* h_src_ptrs: host array [n_layers * n_src] of DEVICE pointers, layer-major
  *             (h_src_ptrs[l * n_src + s] = rows of source s, layer l); row stride = ld elements.
  * d_out     : device int8 [n_dom, out_stride], out_stride >= n_layers*n*m.
- * Launches: 1 memset + (unless TABLES_RESIDENT) 1 H2D copy of the plan tables + 1 kernel. */
+ * Launches: 1 memset + (unless TABLES_RESIDENT) 1 H2D copy of the plan tables + 1 kernel.
+ * Returns DCTD_ERR_UNSUPPORTED, with nothing written to d_out, when the general kernel's shared memory for (D, n, m)
+ * (dynamic layout plus its static variables) exceeds the device's opt-in per-block limit, or when not one of its CTAs
+ * fits on an SM.  The layout grows with D, n and m: on a B200 (232 448 B per block) at n = 3, m = 80 without fusion the
+ * widest supported D is 5068, so D = 5120 (ESM-2 15B) is unsupported.  A fused protein needs a little more. */
 int dctd_fp_execute(const dctd_fp_plan *plan, const void *const *h_src_ptrs, int64_t ld,
                     int8_t *d_out, int64_t out_stride, void *d_workspace, size_t workspace_bytes,
                     uint32_t flags, void *stream);
