@@ -94,6 +94,9 @@ def lib():
         'dctd_l1_pair_scores': (C.c_int, [vp, i32, vp, vp, vp, i64, vp, vp, vp]),
         'dctd_l1_protein_scores_workspace_bytes': (sz, [i64, i64, i64, i64, i32]),
         'dctd_l1_protein_scores': (C.c_int, [vp, vp, i64, vp, vp, i64, i32, vp, vp, vp, sz, vp]),
+        'dctd_l1_protein_hits_workspace_bytes': (sz, [i64, i64, i64, i64, i32, i32, i32]),
+        'dctd_l1_protein_hits': (C.c_int, [vp, vp, i64, vp, vp, i64, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, sz,
+                                           vp]),
     }
     hooks = {'dctd_fp_set_variant', 'dctd_fp_timing_read', 'dctd_l1_set_mode', 'dctd_l1_stream_stamps'}   # tuning builds only
     for name, (res, args) in sig.items():

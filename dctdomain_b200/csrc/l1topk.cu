@@ -277,8 +277,14 @@ __device__ __forceinline__ bool tile_has_flag(const ScanParams &p, long long q0,
 // heap scan: exact top-k with warp-private candidate buffers (any database size; also computes the
 // threshold sample and the fallback for queries whose candidate list overflowed)
 // ------------------------------------------------------------------------------------------
-template <int TQ, int kTD, int STAGES>
-__global__ void __launch_bounds__((kWarps + 1) * 32, 1) l1_scan_kernel(const ScanParams p) {
+// Key policy of the heap scan.  The search orders by the plain key dist << 40 | position; a policy with kClamped set
+// (ClampedKey, l1_hits.cuh) rewrites each tile's distances before selection and counts the keys within a cut.
+struct PlainKey {
+    static constexpr bool kClamped = false;
+};
+
+template <int TQ, int kTD, int STAGES, class Key>
+__device__ __forceinline__ void heap_scan(const ScanParams &p, const Key &key) {
     constexpr int QT = kWarps * TQ;
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ int s_any;
@@ -320,6 +326,16 @@ __global__ void __launch_bounds__((kWarps + 1) * 32, 1) l1_scan_kernel(const Sca
     unsigned int tdist[TQ];      // distance part of each query's current k-th key (fast reject)
 #pragma unroll
     for (int a = 0; a < TQ; ++a) tdist[a] = 0xffffffffu;
+    unsigned int ncut[TQ];       // kClamped: keys within key.cut that this lane saw
+    bool qempty[TQ];
+    if constexpr (Key::kClamped) {
+#pragma unroll
+        for (int a = 0; a < TQ; ++a) {
+            const long long qi = q0 + warp * TQ + a;
+            ncut[a] = 0u;
+            qempty[a] = qi >= p.nq || key.q_empty[qi];
+        }
+    }
 
     for (int t = 0; t < n_tiles; ++t) {
         const int s = t % STAGES;
@@ -328,6 +344,7 @@ __global__ void __launch_bounds__((kWarps + 1) * 32, 1) l1_scan_kernel(const Sca
         sad_tile<TQ, kTD>(reinterpret_cast<const uint4 *>(st + (size_t)s * tile_bytes), qs4, C, lane, acc);
         __syncwarp();
         if (lane == 0) mbar_arrive(&empty[s]);     // this warp no longer reads the stage
+        if constexpr (Key::kClamped) key.template adjust<TQ, kTD>(p, acc, qempty, ncut, g_begin + (long long)t * kTD, g_end, lane);
 
         // ---- candidate filter (warp-private buffers: no CTA-level synchronisation) ----
         bool hit = false;
@@ -371,6 +388,12 @@ __global__ void __launch_bounds__((kWarps + 1) * 32, 1) l1_scan_kernel(const Sca
             for (int i = lane; i < p.k; i += 32) out[i] = (i < keep) ? b[i] : kKeyMax;
         }
     }
+    if constexpr (Key::kClamped) key.template publish<TQ>(ncut, q0 + warp * TQ, p.nq, lane);
+}
+
+template <int TQ, int kTD, int STAGES>
+__global__ void __launch_bounds__((kWarps + 1) * 32, 1) l1_scan_kernel(const ScanParams p) {
+    heap_scan<TQ, kTD, STAGES>(p, PlainKey{});
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1445,6 +1468,8 @@ bool make_bound_plan(const DevInfo &di, long long nq, long long n, int d, int k_
     return true;
 }
 
+#include "l1_hits.cuh"
+
 }  // namespace
 
 extern "C" {
@@ -1734,6 +1759,46 @@ int dctd_l1_protein_scores(const int8_t *d_qf, const int64_t *h_qoff, int64_t n_
         return DCTD_ERR_NOMEM;
     }
     return DCTD_OK;
+}
+
+/* dct-sim database-search hits: see dctd.h */
+static int hits_args(const int64_t *h_qoff, int64_t n_qprot, const int64_t *h_doff, int64_t n_dbprot, int32_t d,
+                     int32_t dist_clamp, int32_t cap) {
+    if (n_qprot < 0 || n_dbprot < 0 || d < 1 || cap < 1 || dist_clamp < 0 || dist_clamp >= (1 << 24)) return DCTD_ERR_ARG;
+    if (!h_qoff || !h_doff || h_qoff[0] != 0 || h_doff[0] != 0) return DCTD_ERR_ARG;
+    for (int64_t a = 0; a < n_qprot; ++a) if (h_qoff[a + 1] < h_qoff[a]) return DCTD_ERR_ARG;
+    for (int64_t b = 0; b < n_dbprot; ++b) if (h_doff[b + 1] < h_doff[b]) return DCTD_ERR_ARG;
+    if (cap > kHitsMaxCap || d > 2048 || n_dbprot >= (1LL << kIdBits)) return DCTD_ERR_UNSUPPORTED;
+    return DCTD_OK;
+}
+
+size_t dctd_l1_protein_hits_workspace_bytes(int64_t n_qf, int64_t n_qprot, int64_t n_dbf, int64_t n_dbprot, int32_t d,
+                                            int32_t top, int32_t cap) {
+    (void)top;
+    if (n_qf < 0 || n_qprot < 0 || n_dbf < 0 || n_dbprot < 0 || d < 1 || cap < 1 || cap > kHitsMaxCap) return 0;
+    DevInfo di;
+    dev_info(&di);
+    HitsLayout l;
+    if (!hits_layout(di, n_qprot, n_dbprot, d, cap, std::max<long long>(1, std::min<long long>(n_qprot, kHitsMaxChunk)), &l))
+        return 0;
+    return l.total;
+}
+
+int dctd_l1_protein_hits(const int8_t *d_qf, const int64_t *h_qoff, int64_t n_qprot, const int8_t *d_dbf,
+                         const int64_t *h_doff, int64_t n_dbprot, int32_t d, int32_t top, int32_t dist_clamp,
+                         int32_t dist_cut, int32_t cap, int32_t *d_count, int32_t *d_hit_db, int32_t *d_hit_min,
+                         int32_t *d_hit_last, void *d_workspace, size_t workspace_bytes, void *stream) {
+    int rc = hits_args(h_qoff, n_qprot, h_doff, n_dbprot, d, dist_clamp, cap);
+    if (rc != DCTD_OK) return rc;
+    if (n_qprot == 0) return DCTD_OK;
+    if (!d_count || !d_hit_db || !d_hit_min || !d_hit_last) return DCTD_ERR_ARG;
+    if ((h_qoff[n_qprot] > 0 && !d_qf) || (h_doff[n_dbprot] > 0 && !d_dbf)) return DCTD_ERR_ARG;
+    try {
+        return run_hits(d_qf, h_qoff, n_qprot, d_dbf, h_doff, n_dbprot, d, top, dist_clamp, dist_cut, cap, d_count,
+                        d_hit_db, d_hit_min, d_hit_last, d_workspace, workspace_bytes, (cudaStream_t)stream);
+    } catch (const std::bad_alloc &) {
+        return DCTD_ERR_NOMEM;
+    }
 }
 
 }  // extern "C"

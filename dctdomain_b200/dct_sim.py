@@ -1,7 +1,9 @@
 """Drop-in for reference ``src/dct-sim.py``: same functions, flags and output text; the L1
-distances come from the GPU - listed pairs through dctd_l1_pair_scores, the all-pairs loops of ``--db`` and all-vs-all
-through dctd_l1_protein_scores (the tiled SAD kernel of the search path) - the float64 similarity formula
-``1 - min(d / 17000, 1)`` (dct-sim.py:23-26) is applied on the host exactly as the reference does.
+distances come from the GPU - listed pairs through dctd_l1_pair_scores, the hits of ``--db`` through
+dctd_l1_protein_hits (a search of each query's global fingerprint against the database's, then the min over fingerprint
+pairs of the selected hits only), all-vs-all through dctd_l1_protein_scores (the tiled SAD kernel of the search path) -
+the float64 similarity formula ``1 - min(d / 17000, 1)`` (dct-sim.py:23-26) is applied on the host exactly as the
+reference does.
 
     python -m dctdomain_b200.dct_sim --dct x-dct.npz --pair x.pair --output x-dctsim.txt
 """
@@ -80,6 +82,101 @@ def protein_scores(q_fps, q_off, db_fps, db_off, workspace_bytes: int = None):
             return m1.reshape(nq, nd), l1.reshape(nq, nd)
         _lib.check(rc, 'dctd_l1_protein_scores')
     return mn.cpu().numpy().astype(np.int64), last.cpu().numpy().astype(np.int64)
+
+
+DIST_CLAMP = 17000                 # s(x) = 1 - min(x / 17000, 1) is 0 for every x >= 17000
+HITS_MAX_CAP = 992                 # longest hit row dctd_l1_protein_hits fills
+
+
+def _dist_cut(threshold: float) -> int:
+    """The largest distance x whose similarity passes dct-sim's threshold (s(x) >= threshold), found by evaluating the
+    float64 expression itself over 0 .. 17000 (it is strictly decreasing there).  -1: nothing passes; DIST_CLAMP: every
+    database protein passes, those without fingerprints included (threshold <= 0, or NaN: ``s < nan`` never ends
+    dct-sim's loop)."""
+    threshold = float(threshold)
+    if threshold != threshold:
+        return DIST_CLAMP
+    x = np.arange(DIST_CLAMP + 1, dtype=np.int64)
+    ok = np.nonzero(1.0 - np.minimum(x / 17000, 1.0) >= threshold)[0]
+    return int(ok[-1]) if len(ok) else -1
+
+
+def protein_hits(q_fps, q_off, db_fps, db_off, top: int, threshold: float, cap: int = None,
+                 workspace_bytes: int = None):
+    """dct-sim's database-search hits (src/dct-sim.py:126-156) without the all-pairs matrices: for query protein a, the
+    database proteins ranked by the similarity of the two proteins' last (global) fingerprints - ascending by
+    (min(last, 17000), b) - cut after max(top, #{b : s(last) >= threshold}) entries, exactly the rows dct-sim prints.
+    Returns CSR int arrays (hit_off [n_q + 1], hit_db, hit_min, hit_last): hits of query a are
+    hit_off[a] .. hit_off[a+1]-1 in output order, with the min over all fingerprint pairs and the last-vs-last distance
+    (INT32_MAX where a protein has no fingerprints).
+
+    One dctd_l1_protein_hits call with rows of ``cap`` hits (default max(top, 32)); queries with more hits than that are
+    rerun once with cap = their largest count.  Raises DctdError(ERR_UNSUPPORTED) where the device path cannot give the
+    rows: vectors too wide for its tiles, or more than HITS_MAX_CAP hits for one query."""
+    dev = _device()
+    L = _lib.lib()
+    q_off = np.ascontiguousarray(q_off, dtype=np.int64)
+    db_off = np.ascontiguousarray(db_off, dtype=np.int64)
+    nq, nd = len(q_off) - 1, len(db_off) - 1
+    d_q = q_fps if isinstance(q_fps, torch.Tensor) else torch.from_numpy(_as_int8(q_fps)).to(dev)
+    d_db = db_fps if isinstance(db_fps, torch.Tensor) else torch.from_numpy(_as_int8(db_fps)).to(dev)
+    d_q, d_db = d_q.contiguous(), d_db.contiguous()
+    d = int(d_q.shape[1]) if d_q.dim() == 2 and d_q.shape[0] else int(d_db.shape[1])
+    top_ = min(max(int(top), 0), nd)
+    cut = _dist_cut(threshold)
+    if cap is None:
+        cap = max(top_, 32)
+    if cap > HITS_MAX_CAP:
+        raise _lib.DctdError(_lib.ERR_UNSUPPORTED, f'protein_hits: {cap} hits per query (at most {HITS_MAX_CAP})')
+
+    def run(q, qoff, cap):
+        n = len(qoff) - 1
+        count = torch.empty(n, dtype=torch.int32, device=dev)
+        rows = torch.empty((3, n, cap), dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            need = workspace_bytes or int(L.dctd_l1_protein_hits_workspace_bytes(int(q.shape[0]), n, int(d_db.shape[0]),
+                                                                                 nd, d, top_, cap))
+            ws = torch.empty(max(need, 256), dtype=torch.uint8, device=dev)
+            rc = L.dctd_l1_protein_hits(q.data_ptr(), qoff.ctypes.data, n, d_db.data_ptr(), db_off.ctypes.data, nd, d,
+                                        top_, DIST_CLAMP, cut, cap, count.data_ptr(), rows[0].data_ptr(),
+                                        rows[1].data_ptr(), rows[2].data_ptr(), ws.data_ptr(), ws.numel(), stream)
+        _lib.check(rc, 'dctd_l1_protein_hits')
+        return count.cpu().numpy().astype(np.int64), rows.cpu().numpy()
+
+    def scatter(out, off, count, rows, sel):
+        """rows of the queries `sel` -> their CSR slots"""
+        width = rows.shape[2]
+        m = np.arange(width)[None, :] < count[sel][:, None]
+        pos = (off[:-1][sel][:, None] + np.arange(width)[None, :])[m]
+        for o, r in zip(out, rows[:, sel]):
+            o[pos] = r[m]
+
+    if nq == 0:
+        count, rows = np.zeros(0, dtype=np.int64), np.zeros((3, 0, cap), dtype=np.int32)
+    else:
+        count, rows = run(d_q, q_off, cap)
+    off = np.concatenate([[0], np.cumsum(count)]).astype(np.int64)
+    out = [np.empty(int(off[-1]), dtype=np.int64) for _ in range(3)]
+    scatter(out, off, count, rows, count <= cap)
+    over = np.nonzero(count > cap)[0]
+    if len(over):                          # longer hit lists: one more call for those queries only
+        cap2 = int(count[over].max())
+        if cap2 > HITS_MAX_CAP:
+            raise _lib.DctdError(_lib.ERR_UNSUPPORTED, f'protein_hits: {cap2} hits for one query (at most {HITS_MAX_CAP})')
+        lens = q_off[over + 1] - q_off[over]
+        sub_off = np.concatenate([[0], np.cumsum(lens)]).astype(np.int64)
+        idx = np.concatenate([np.arange(q_off[a], q_off[a + 1]) for a in over]).astype(np.int64)
+        sub_q = d_q[torch.from_numpy(idx).to(dev)] if len(idx) else d_q[:0]
+        count2, rows2 = run(sub_q.contiguous(), sub_off, cap2)
+        full = np.zeros(nq, dtype=bool)
+        full[over] = True
+        rows_full = np.zeros((3, nq, cap2), dtype=np.int32)
+        rows_full[:, over] = rows2
+        count_full = count.copy()
+        count_full[over] = count2
+        scatter(out, off, count_full, rows_full, full)
+    return off, out[0], out[1], out[2]
 
 
 def _sim(dist):
@@ -182,6 +279,18 @@ def db_search(npzfile: str, dbfile: str, top: int, threshold: float, output: str
     nq, nd = len(seqid), len(db_seqid)
     qcat, qoff = _blocks(list(dct))
     dcat, doff = _blocks(list(db_dct))
+    try:
+        off, hit_db, hit_min, hit_last = protein_hits(qcat, qoff, dcat, doff, top, threshold)
+    except _lib.DctdError as e:
+        if e.code != _lib.ERR_UNSUPPORTED:
+            raise
+    else:
+        for i in range(nq):
+            for j in range(off[i], off[i + 1]):
+                maxs, s = _maxs_s(hit_min[j], hit_last[j])
+                _emit(f"{seqid[i]} {db_seqid[hit_db[j]]} {maxs} {s}", output)
+        return
+    # wide fingerprints or very long hit lists: score all pairs
     mn, last = protein_scores(qcat, qoff, dcat, doff)            # all pairs: one tiled pass on the device
     # the reference sorts every query's hits by the global similarity, descending and stable (sorted(..., reverse=True)
     # keeps the database order among equal keys), and prints until rank >= top and s < threshold

@@ -254,6 +254,31 @@ int dctd_l1_protein_scores(const int8_t *d_qf, const int64_t *h_qoff, int64_t n_
                            const int64_t *h_doff, int64_t n_dbprot, int32_t d, int32_t *d_min_dist,
                            int32_t *d_last_dist, void *d_workspace, size_t workspace_bytes, void *stream);
 
+/* The HITS of dct-sim's database search (src/dct-sim.py:126-156) without the [n_qprot, n_dbprot] matrices above: per
+ * query protein a, database proteins in ascending order of the clamped key (min(last(a,b), dist_clamp), b), where
+ * last(a,b) is the L1 distance of the two proteins' LAST fingerprint rows (dist_clamp when either protein has none).
+ * That is dct-sim's stable descending sort on s = 1 - min(last / 17000, 1) with dist_clamp = 17000.  The hits of a are
+ * the first count[a] = max(top', c_a) entries of that order, top' = min(max(top, 0), n_dbprot) and
+ * c_a = #{b : min(last(a,b), dist_clamp) <= dist_cut} (dist_cut < 0: none; dist_cut >= dist_clamp: all).
+ *   d_qf, d_dbf   device int8 row-major fingerprints; protein a owns rows h_qoff[a] .. h_qoff[a+1]-1 of d_qf, protein b
+ *                 rows h_doff[b] .. h_doff[b+1]-1 of d_dbf (HOST offsets starting at 0)
+ *   d_count       device int32 [n_qprot]: count[a], exact whatever cap is
+ *   d_hit_db, d_hit_min, d_hit_last   device int32 [n_qprot, cap]: row a holds the first min(count[a], cap) hits in
+ *                 order - database protein, min over all fingerprint pairs, last-vs-last distance (INT32_MAX when
+ *                 either protein has no fingerprints) - and (-1, INT32_MAX, INT32_MAX) after them
+ * One SAD per (query protein, database protein) pair selects the hits (heap scan of the search path with the clamped
+ * key); the min is computed for the hit pairs only.  Query proteins are processed in as many chunks as the workspace
+ * allows (dctd_l1_protein_hits_workspace_bytes: one chunk of up to 65536 of them).  1 <= cap <= 992;
+ * DCTD_ERR_UNSUPPORTED for cap > 992 (a caller that needs longer rows reruns those queries through
+ * dctd_l1_protein_scores) and for vectors too wide for the shared-memory tiles (d > ~1000).  Arguments are checked
+ * before any CUDA call. */
+size_t dctd_l1_protein_hits_workspace_bytes(int64_t n_qf, int64_t n_qprot, int64_t n_dbf, int64_t n_dbprot, int32_t d,
+                                            int32_t top, int32_t cap);
+int dctd_l1_protein_hits(const int8_t *d_qf, const int64_t *h_qoff, int64_t n_qprot, const int8_t *d_dbf,
+                         const int64_t *h_doff, int64_t n_dbprot, int32_t d, int32_t top, int32_t dist_clamp,
+                         int32_t dist_cut, int32_t cap, int32_t *d_count, int32_t *d_hit_db, int32_t *d_hit_min,
+                         int32_t *d_hit_last, void *d_workspace, size_t workspace_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
