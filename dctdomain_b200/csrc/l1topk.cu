@@ -286,13 +286,15 @@ struct PlainKey {
 template <int TQ, int kTD, int STAGES, class Key>
 __device__ __forceinline__ void heap_scan(const ScanParams &p, const Key &key) {
     constexpr int QT = kWarps * TQ;
+    // no static shared memory: make_config gives the dynamic part everything up to the opt-in limit (d = 833..848 leaves
+    // 96 B), and even one static int takes 128 B next to the 128-B aligned dynamic array
     extern __shared__ __align__(128) unsigned char smem[];
-    __shared__ int s_any;
     const int C = chunks_of(p.d);
     const int dpad = C * 16;
     const int tile_bytes = kTD * 32 * dpad;
     unsigned long long *full = reinterpret_cast<unsigned long long *>(smem);           // [STAGES]
     unsigned long long *empty = full + STAGES;                                          // [STAGES]
+    int *s_any = reinterpret_cast<int *>(empty + STAGES);                               // tile_has_flag
     unsigned char *qs = smem + 128;                                                     // [QT][dpad]
     unsigned char *st = qs + (size_t)QT * dpad;                                         // [STAGES][tile]
     unsigned long long *buf = reinterpret_cast<unsigned long long *>(st + (size_t)STAGES * tile_bytes);
@@ -301,7 +303,7 @@ __device__ __forceinline__ void heap_scan(const ScanParams &p, const Key &key) {
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const long long q0 = (long long)blockIdx.y * QT;
-    if (p.qflags && !tile_has_flag(p, q0, QT, &s_any)) return;
+    if (p.qflags && !tile_has_flag(p, q0, QT, s_any)) return;
     const long long g_begin = (long long)blockIdx.x * p.groups_per_split;
     const long long g_end = min(p.n_groups, g_begin + p.groups_per_split);
     const int n_tiles = (int)((g_end - g_begin + kTD - 1) / kTD);

@@ -109,7 +109,7 @@ def _check(got, want):
         assert g.dtype == np.int64 and np.array_equal(g, w), (name, g[:20], w[:20])
 
 
-@pytest.mark.parametrize('d', [480, 100, 16])
+@pytest.mark.parametrize('d', [480, 100, 16, 840])       # 840: the heap scan's shared memory at the opt-in limit
 def test_hits_match_dct_sim_rule(d):
     from dctdomain_b200 import dct_sim
     qf, qoff, df, doff = _dataset(d, 45, 201, d)           # 201: the database is not a multiple of 32
