@@ -91,6 +91,8 @@ def lib():
         'dctd_l1_uses_bound': (C.c_int, [i64, i64, i32, i32]),
         'dctd_l1_topk_keys': (C.c_int, [vp, i64, vp, i64, i32, i32, i64, vp, vp, vp, sz, u32, vp]),
         'dctd_l1_keys_merge': (C.c_int, [vp, i32, i64, i32, vp, vp, vp, vp]),
+        'dctd_l1_topk_large_workspace_bytes': (sz, [i64, i64, i32, i32]),
+        'dctd_l1_topk_large': (C.c_int, [vp, i64, vp, i64, i32, i32, i64, vp, vp, vp, vp, sz, vp]),
         'dctd_l1_pair_scores': (C.c_int, [vp, i32, vp, vp, vp, i64, vp, vp, vp]),
         'dctd_l1_protein_scores_workspace_bytes': (sz, [i64, i64, i64, i64, i32]),
         'dctd_l1_protein_scores': (C.c_int, [vp, vp, i64, vp, vp, i64, i32, vp, vp, vp, sz, vp]),

@@ -1471,6 +1471,7 @@ bool make_bound_plan(const DevInfo &di, long long nq, long long n, int d, int k_
 }
 
 #include "l1_hits.cuh"
+#include "l1_large.cuh"
 
 }  // namespace
 
@@ -1597,13 +1598,14 @@ int dctd_l1_bound(const int8_t *d_q, int64_t nq, const void *d_packed, int64_t n
 
 int dctd_l1_topk_merge(const float *d_dist_parts, const int64_t *d_ids_parts, int32_t parts, int64_t nq,
                        int32_t k, float *d_dist, int64_t *d_ids, void *stream) {
-    if (parts < 1 || parts > 1024 || nq < 0 || k < 1 || k > 1024) return DCTD_ERR_ARG;
+    if (parts < 1 || parts > 1024 || nq < 0 || k < 1 || k > kLargeMaxK) return DCTD_ERR_ARG;
     if (nq == 0) return DCTD_OK;
     if (!d_dist_parts || !d_ids_parts || !d_dist || !d_ids) return DCTD_ERR_ARG;
     MergeParams mp{};
     mp.dist_parts = d_dist_parts; mp.id_parts = (const long long *)d_ids_parts;
     mp.parts = parts; mp.ppw = parts; mp.nq = nq; mp.k = k; mp.cap = next_pow2(2 * k); mp.id_base = 0;
     mp.dist = d_dist; mp.ids = (long long *)d_ids;
+    if (k > 992) return run_rank_merge(mp, true, (cudaStream_t)stream);
     const int warps = 4;
     const size_t msmem = (size_t)warps * mp.cap * 8;
     DCTD_CUDA_TRY(cudaFuncSetAttribute(l1_merge_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem));
@@ -1614,11 +1616,30 @@ int dctd_l1_topk_merge(const float *d_dist_parts, const int64_t *d_ids_parts, in
 
 int dctd_l1_keys_merge(const uint64_t *d_key_parts, int32_t parts, int64_t nq, int32_t k, float *d_dist,
                        int64_t *d_ids, uint64_t *d_keys, void *stream) {
-    if (parts < 1 || parts > kMergePPW || nq < 0 || k < 1 || k > 1024) return DCTD_ERR_ARG;
+    if (parts < 1 || parts > kMergePPW || nq < 0 || k < 1 || k > kLargeMaxK) return DCTD_ERR_ARG;
     if (nq == 0) return DCTD_OK;
     if (!d_key_parts || ((!d_dist || !d_ids) && !d_keys) || ((d_dist == nullptr) != (d_ids == nullptr))) return DCTD_ERR_ARG;
+    if (k > 992) {
+        MergeParams mp{};
+        mp.key_parts = (const unsigned long long *)d_key_parts; mp.parts = parts; mp.nq = nq; mp.k = k;
+        mp.dist = d_dist; mp.ids = (long long *)d_ids; mp.key_out = (unsigned long long *)d_keys;
+        return run_rank_merge(mp, false, (cudaStream_t)stream);
+    }
     return run_merge((const unsigned long long *)d_key_parts, parts, nq, k, 0, d_dist, (long long *)d_ids,
                      (unsigned long long *)d_keys, nullptr, nullptr, (cudaStream_t)stream);
+}
+
+size_t dctd_l1_topk_large_workspace_bytes(int64_t nq, int64_t n, int32_t d, int32_t k) {
+    LargeLayout l;
+    if (n < 0 || !large_layout(nq, d, k, &l)) return 0;
+    return l.total;
+}
+
+int dctd_l1_topk_large(const int8_t *d_q, int64_t nq, const void *d_packed, int64_t n, int32_t d, int32_t k,
+                       int64_t id_base, float *d_dist, int64_t *d_ids, uint64_t *d_keys, void *d_workspace,
+                       size_t workspace_bytes, void *stream) {
+    return run_topk_large(d_q, nq, d_packed, n, d, k, id_base, d_dist, (long long *)d_ids, (unsigned long long *)d_keys,
+                          d_workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int dctd_l1_pair_scores(const int8_t *d_fps, int32_t d, const int64_t *d_off, const int32_t *d_pair_a,

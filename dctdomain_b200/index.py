@@ -32,6 +32,8 @@ METRIC_L1 = 2
 
 FLT_MAX = float(np.finfo(np.float32).max)
 _QUERY_BATCH = 8192     # queries per dctd_l1_topk call (bounds the candidate workspace: 64 KB per query)
+K_HEAP_MAX = 992        # largest k of dctd_l1_topk / dctd_l1_topk_keys; larger k go to dctd_l1_topk_large
+K_MAX = 8192            # largest k of dctd_l1_topk_large
 
 
 def _as_int8(x, d=None) -> np.ndarray:
@@ -120,6 +122,9 @@ class IndexFlat:
         nq = int(q.shape[0])
         dist = torch.empty((nq, k), dtype=torch.float32, device=self._dev)
         ids = torch.empty((nq, k), dtype=torch.int64, device=self._dev)
+        if k > K_HEAP_MAX:
+            self._topk_large(q, k, id_base, dist=dist, ids=ids)
+            return dist, ids
         packed_ptr = self._packed.data_ptr() if self._packed is not None else 0
         with torch.cuda.device(self._dev):
             stream = torch.cuda.current_stream(self._dev).cuda_stream
@@ -127,7 +132,7 @@ class IndexFlat:
                 e = min(nq, b + _QUERY_BATCH)
                 need = int(L.dctd_l1_topk_workspace_bytes(e - b, self.ntotal, self.d, k))
                 if need == 0:
-                    raise _lib.DctdError(_lib.ERR_UNSUPPORTED, f'k={k}, d={self.d} not supported (k <= 992, d <= 2048)')
+                    raise _lib.DctdError(_lib.ERR_UNSUPPORTED, f'k={k}, d={self.d} not supported (k <= {K_MAX}, d <= 2048)')
                 ws = _workspace(self._dev, need)
                 rc = L.dctd_l1_topk(q[b:e].data_ptr(), e - b, packed_ptr, self.ntotal, self.d, k, id_base,
                                     dist[b:e].data_ptr(), ids[b:e].data_ptr(), ws.data_ptr(), ws.numel(), stream)
@@ -180,6 +185,11 @@ class IndexFlat:
         q = q.contiguous()
         nq = int(q.shape[0])
         keys = torch.empty((nq, k), dtype=torch.int64, device=self._dev)
+        if k > K_HEAP_MAX:
+            if bound is not None or heap_only:
+                raise ValueError(f'bound and heap_only apply to k <= {K_HEAP_MAX} only')
+            self._topk_large(q, k, id_base, keys=keys)
+            return keys
         if bound is not None:
             if bound.dtype != torch.int32 or bound.shape != (nq,) or not bound.is_cuda:
                 raise ValueError('bound must be an int32 CUDA tensor [nq]')
@@ -191,13 +201,33 @@ class IndexFlat:
                 e = min(nq, b + _QUERY_BATCH)
                 need = int(L.dctd_l1_topk_workspace_bytes(e - b, self.ntotal, self.d, k))
                 if need == 0:
-                    raise _lib.DctdError(_lib.ERR_UNSUPPORTED, f'k={k}, d={self.d} not supported (k <= 992, d <= 2048)')
+                    raise _lib.DctdError(_lib.ERR_UNSUPPORTED, f'k={k}, d={self.d} not supported (k <= {K_MAX}, d <= 2048)')
                 ws = _workspace(self._dev, need)
                 rc = L.dctd_l1_topk_keys(q[b:e].data_ptr(), e - b, packed_ptr, self.ntotal, self.d, k, id_base,
                                          bound[b:e].data_ptr() if bound is not None else 0, keys[b:e].data_ptr(),
                                          ws.data_ptr(), ws.numel(), _lib.L1_HEAP_ONLY if heap_only else 0, stream)
                 _lib.check(rc, 'dctd_l1_topk_keys')
         return keys
+
+    def _topk_large(self, q, k, id_base, dist=None, ids=None, keys=None):
+        """k > K_HEAP_MAX: dctd_l1_topk_large (radix selection) into (dist, ids) or keys."""
+        if k > K_MAX:
+            raise _lib.DctdError(_lib.ERR_UNSUPPORTED, f'k={k} not supported (k <= {K_MAX})')
+        L = _lib.lib()
+        nq = int(q.shape[0])
+        packed_ptr = self._packed.data_ptr() if self._packed is not None else 0
+        with torch.cuda.device(self._dev):
+            stream = torch.cuda.current_stream(self._dev).cuda_stream
+            for b in range(0, nq, _QUERY_BATCH):
+                e = min(nq, b + _QUERY_BATCH)
+                need = int(L.dctd_l1_topk_large_workspace_bytes(e - b, self.ntotal, self.d, k))
+                if need == 0:
+                    raise _lib.DctdError(_lib.ERR_UNSUPPORTED, f'k={k}, d={self.d} not supported (k <= {K_MAX}, d <= 2048)')
+                ws = _workspace(self._dev, need)
+                ptr = lambda t: t[b:e].data_ptr() if t is not None else 0   # noqa: E731
+                rc = L.dctd_l1_topk_large(q[b:e].data_ptr(), e - b, packed_ptr, self.ntotal, self.d, k, id_base, ptr(dist),
+                                          ptr(ids), ptr(keys), ws.data_ptr(), ws.numel(), stream)
+                _lib.check(rc, 'dctd_l1_topk_large')
 
     def search(self, x, k: int):
         """faiss-style ``D, I = index.search(x, k)`` with host arrays."""

@@ -218,17 +218,33 @@ int dctd_l1_uses_bound(int64_t nq, int64_t n, int32_t d, int32_t k);
 int dctd_l1_topk_keys(const int8_t *d_q, int64_t nq, const void *d_packed, int64_t n, int32_t d, int32_t k,
                       int64_t id_base, const int32_t *d_bound, uint64_t *d_keys, void *d_workspace,
                       size_t workspace_bytes, uint32_t flags, void *stream);
-/* d_key_parts uint64 [parts, nq, k] (parts <= 32), each list ascending -> the k smallest keys per query as
+/* d_key_parts uint64 [parts, nq, k] (parts <= 32, k <= 8192), each list ascending -> the k smallest keys per query as
  * (d_dist float32 [nq, k], d_ids int64 [nq, k]) with (FLT_MAX, -1) padding and / or as keys (d_keys, may be NULL;
- * d_dist and d_ids may both be NULL when d_keys is given) */
+ * d_dist and d_ids may both be NULL when d_keys is given).  k > 992 merges by rank (no shared memory). */
 int dctd_l1_keys_merge(const uint64_t *d_key_parts, int32_t parts, int64_t nq, int32_t k, float *d_dist,
                        int64_t *d_ids, uint64_t *d_keys, void *stream);
 
 /* k-way merge of `parts` sorted lists: d_dist_parts float32 [parts, nq, k], d_ids_parts int64
- * [parts, nq, k] (each ascending by (dist, id), padded with (FLT_MAX, -1)) -> [nq, k].
+ * [parts, nq, k] (each ascending by (dist, id), padded with (FLT_MAX, -1)) -> [nq, k], k <= 8192.
  * Used after the NCCL all-gather of the per-rank results of a sharded database. */
 int dctd_l1_topk_merge(const float *d_dist_parts, const int64_t *d_ids_parts, int32_t parts,
                        int64_t nq, int32_t k, float *d_dist, int64_t *d_ids, void *stream);
+
+/* ---- large k: 1 <= k <= 8192 (dctd_l1_topk / dctd_l1_topk_keys stop at k = 992).  The same result as those two -
+ * faiss' (d_dist float32 [nq, k], d_ids int64 [nq, k]) with (FLT_MAX, -1) padding past n, and / or (d_keys uint64
+ * [nq, k], may be NULL; d_dist and d_ids both NULL or both set) the packed keys distance << 40 | id_base + position with
+ * UINT64_MAX padding - by radix selection instead of a heap: per query, histogram passes over the database narrow a
+ * window of the key space to one holding the k-th key with at most 16384 keys at or below it (normally one pass), one
+ * more pass collects those keys and they are sorted.  n <= 16384: one pass collects everything.
+ * Queries are processed in chunks of 2048; the workspace (dctd_l1_topk_large_workspace_bytes, 0 for an unsupported k or
+ * d) is ~130 KB per query of one chunk, ~270 MB from 2048 queries upwards, whatever n is.
+ * DCTD_ERR_UNSUPPORTED for k > 8192 or d > 2048; arguments are checked before any CUDA call.  When the call's work has
+ * completed, the first 4 bytes of the workspace hold, as uint32, the number of histogram passes the call needed: the
+ * most any query took part in (0 for n <= 16384). */
+size_t dctd_l1_topk_large_workspace_bytes(int64_t nq, int64_t n, int32_t d, int32_t k);
+int dctd_l1_topk_large(const int8_t *d_q, int64_t nq, const void *d_packed, int64_t n, int32_t d, int32_t k,
+                       int64_t id_base, float *d_dist, int64_t *d_ids, uint64_t *d_keys, void *d_workspace,
+                       size_t workspace_bytes, void *stream);
 
 /* Pairwise scorer of reference src/dct-sim.py:12-50: for pair p, the int L1 distances of every
  * fingerprint of protein a[p] against every fingerprint of protein b[p] (rows
