@@ -886,6 +886,7 @@ __global__ void __launch_bounds__(128) l1_merge_kernel(const MergeParams p) {
 // ------------------------------------------------------------------------------------------
 // VEC16: d is a multiple of 16 and the rows are 16-byte aligned -> lane c reads chunk c of both fingerprints as one
 // uint4 and takes four packed-byte SADs (bytes biased by 0x80 so that the unsigned SAD is |a - b| for int8)
+// A pair with an empty side keeps INT32_MAX in both outputs, as dctd_l1_protein_scores and dctd_l1_protein_hits report it.
 template <bool VEC16>
 __global__ void pair_scores_kernel(const int8_t *__restrict__ fps, int d, const long long *__restrict__ off,
                                    const int *__restrict__ pa, const int *__restrict__ pb, long long n_pairs,
@@ -894,7 +895,7 @@ __global__ void pair_scores_kernel(const int8_t *__restrict__ fps, int d, const 
     const long long pr = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (pr >= n_pairs) return;
     const long long a0 = off[pa[pr]], a1 = off[pa[pr] + 1], b0 = off[pb[pr]], b1 = off[pb[pr] + 1];
-    int best = 0x7fffffff, last = 0;
+    int best = 0x7fffffff, last = 0x7fffffff;
     for (long long i = a0; i < a1; ++i)
         for (long long j = b0; j < b1; ++j) {
             int s = 0;

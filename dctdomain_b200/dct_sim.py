@@ -20,7 +20,8 @@ from .fingerprint import _device
 
 
 def _pair_dists(fps: np.ndarray, off: np.ndarray, pa: np.ndarray, pb: np.ndarray):
-    """(min over fingerprint pairs, last-vs-last) int L1 distances for protein pairs (pa[i], pb[i])."""
+    """(min over fingerprint pairs, last-vs-last) int L1 distances for protein pairs (pa[i], pb[i]); INT32_MAX for both
+    where either protein has no fingerprints."""
     dev = _device()
     fps = _as_int8(fps)
     n = len(pa)

@@ -249,7 +249,8 @@ int dctd_l1_topk_large(const int8_t *d_q, int64_t nq, const void *d_packed, int6
 /* Pairwise scorer of reference src/dct-sim.py:12-50: for pair p, the int L1 distances of every
  * fingerprint of protein a[p] against every fingerprint of protein b[p] (rows
  * [off[x], off[x+1]) of d_fps, int8 [n_fps, d] row-major): d_min_dist[p] = min over all
- * fingerprint pairs, d_last_dist[p] = distance of the last-vs-last pair.  The caller turns them
+ * fingerprint pairs, d_last_dist[p] = distance of the last-vs-last pair; both INT32_MAX when either protein has no
+ * fingerprints, as in dctd_l1_protein_scores and dctd_l1_protein_hits.  Any d >= 1.  The caller turns them
  * into similarities (1 - min(dist/17000, 1)) on the host in float64, as the reference does. */
 int dctd_l1_pair_scores(const int8_t *d_fps, int32_t d, const int64_t *d_off, const int32_t *d_pair_a,
                         const int32_t *d_pair_b, int64_t n_pairs, int32_t *d_min_dist,
@@ -264,7 +265,9 @@ int dctd_l1_pair_scores(const int8_t *d_fps, int32_t d, const int64_t *d_off, co
  *   d_min_dist, d_last_dist   device int32 [n_qprot, n_dbprot]; INT32_MAX where a protein has no fingerprints
  * The query proteins are processed in as many chunks as the workspace requires (dctd_l1_protein_scores_workspace_bytes
  * returns a size that keeps the intermediate matrices at <= 1 GB; anything from one tile of queries upwards works).
- * DCTD_ERR_UNSUPPORTED for vectors too wide for the shared-memory tiles (d > ~1000): use dctd_l1_pair_scores. */
+ * DCTD_ERR_UNSUPPORTED, before any launch, for vectors too wide for the shared-memory tiles: the kernel needs
+ * 192 + 384 * dpad bytes (dpad = d rounded up to a multiple of 16), so on a B200 (232 448 B opt-in per block) d <= 592
+ * runs and d >= 593 does not: use dctd_l1_pair_scores there. */
 size_t dctd_l1_protein_scores_workspace_bytes(int64_t n_qf, int64_t n_qprot, int64_t n_dbf, int64_t n_dbprot, int32_t d);
 int dctd_l1_protein_scores(const int8_t *d_qf, const int64_t *h_qoff, int64_t n_qprot, const void *d_db_packed,
                            const int64_t *h_doff, int64_t n_dbprot, int32_t d, int32_t *d_min_dist,
@@ -286,8 +289,7 @@ int dctd_l1_protein_scores(const int8_t *d_qf, const int64_t *h_qoff, int64_t n_
  * key); the min is computed for the hit pairs only.  Query proteins are processed in as many chunks as the workspace
  * allows (dctd_l1_protein_hits_workspace_bytes: one chunk of up to 65536 of them).  1 <= cap <= 992;
  * DCTD_ERR_UNSUPPORTED for cap > 992 (a caller that needs longer rows reruns those queries through
- * dctd_l1_protein_scores) and for vectors too wide for the shared-memory tiles (d > ~1000).  Arguments are checked
- * before any CUDA call. */
+ * dctd_l1_protein_scores) and for d > 2048 (up to 2048 its heap scan fits a B200's shared memory at every cap).  Arguments are checked before any CUDA call. */
 size_t dctd_l1_protein_hits_workspace_bytes(int64_t n_qf, int64_t n_qprot, int64_t n_dbf, int64_t n_dbprot, int32_t d,
                                             int32_t top, int32_t cap);
 int dctd_l1_protein_hits(const int8_t *d_qf, const int64_t *h_qoff, int64_t n_qprot, const int8_t *d_dbf,
